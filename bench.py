@@ -1,6 +1,7 @@
 """bench.py -- collocation-points/sec for one residual+gradient evaluation (BASELINE.json metric) on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2] [--points P] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic collocation points: K0 pack -> K1 (forward jets +
 residual + seeds) -> loss finalize -> K2 (reverse pass) -> K2b (reduce); with N > 1 GPUs every rank owns its own
@@ -52,7 +53,12 @@ def parse():
     ap.add_argument("--no-gpu-comparator", action="store_true", help="skip the torch-CUDA-autograd comparator leg")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--no-strong", action="store_true", help="skip the C3 / C5 strong-scaling legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (grad.npy, sumsq.npy) under DIR")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -345,6 +351,15 @@ def executed_flops(wl, tp):
     return total
 
 
+def dump_outputs(out_dir, fp):
+    """What a caller of the timed step receives, as float32 .npy files: ``grad`` = d mean(r^2) / d theta (flat, in the
+    order of the networks' parameters) and ``sumsq`` = sum r^2 over the global batch.  Inputs are seeded (parameters:
+    seed 0, points: seed 1000 + rank), so two builds given the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "grad.npy"), fp.grad.detach().cpu().numpy())
+    np.save(os.path.join(out_dir, "sumsq.npy"), fp.sumsq.detach().cpu().numpy())
+
+
 def load_peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -473,6 +488,8 @@ def main():
     ms_per_step = total_ms / args.steps
     value = n_global / (ms_per_step * 1e-3)
     loss = float(fp.sumsq.item()) / (n_global * fp.n_eq)
+    if args.dump_outputs and rank == 0:   # before the per-kernel timing below overwrites the gradient
+        dump_outputs(args.dump_outputs, fp)
 
     # ---- per-kernel timing for the roofline (events around each launch, same stream) ---------------------------------
     info = fp.plan_info(n)
@@ -682,7 +699,7 @@ def main():
             "fit": fit, "gpu_autograd_baseline": gpu_cmp,
             "loss": loss, "wall_s_timed_region": t_wall,
             "step_ms_stats": {"min": float(step_ms.min()), "median": float(np.median(step_ms)),
-                              "max": float(step_ms.max())},
+                              "max": float(step_ms.max()), "count": int(step_ms.size)},
         }
         print(json.dumps(line), flush=True)
     if world > 1:

@@ -117,3 +117,39 @@ def test_specialised_kernel_compiles_for_sm_100a(tmp_path, monkeypatch):
     assert data[:4] == b"\x7fELF" and os.path.exists(os.path.join(str(tmp_path), key + ".cubin"))
     data2, key2 = jit.compile_cubin(tp)                                    # second call: served from the cache
     assert key2 == key and data2 == data
+    monkeypatch.setattr(jit, "_cache_dir", lambda: None)                   # no trustworthy cache directory: compile, keep nothing
+    os.remove(os.path.join(str(tmp_path), key + ".cubin"))
+    data3, key3 = jit.compile_cubin(tp)
+    assert key3 == key and data3[:4] == b"\x7fELF" and os.listdir(str(tmp_path)) == []
+
+
+def test_cache_falls_back_to_a_private_temporary_directory(tmp_path, monkeypatch):
+    """A cache directory that cannot be created (no writable home) moves the cubin cache to a per-user directory under the
+    temporary directory, created private.  A cached cubin runs in the caller's CUDA context, so a directory another account
+    could write to -- world-writable, owned by someone else, or a symlink -- is never used: no caching then."""
+    import tempfile
+    from neurodiffeq_b200 import jit
+    blocker = tmp_path / "not_a_directory"
+    blocker.write_text("")
+    monkeypatch.setattr(jit, "CACHE", str(blocker / "pinnjet_jit"))
+    tmp = tmp_path / "tmp"
+    os.makedirs(str(tmp))
+    monkeypatch.setattr(tempfile, "tempdir", str(tmp))
+    fallback = os.path.join(str(tmp), f"pinnjet_jit-{os.getuid()}")
+    assert jit._cache_dir() == fallback and os.stat(fallback).st_mode & 0o077 == 0
+
+    os.chmod(fallback, 0o777)                                              # planted world-writable
+    assert jit._cache_dir() is None
+    os.rmdir(fallback)
+    os.makedirs(str(tmp_path / "elsewhere"), mode=0o700)
+    os.symlink(str(tmp_path / "elsewhere"), fallback)                     # planted symlink
+    assert jit._cache_dir() is None
+    os.remove(fallback)
+    real_uid = os.getuid()
+    monkeypatch.setattr(os, "getuid", lambda: real_uid + 1)               # a private directory of ANOTHER account
+    os.makedirs(os.path.join(str(tmp), f"pinnjet_jit-{real_uid + 1}"), mode=0o700)
+    assert jit._cache_dir() is None
+    monkeypatch.setattr(os, "getuid", lambda: real_uid)
+
+    monkeypatch.setattr(jit, "CACHE", str(tmp_path / "home_cache"))       # a usable CACHE comes first
+    assert jit._cache_dir() == str(tmp_path / "home_cache")
